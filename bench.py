@@ -2,7 +2,7 @@
 """bench.py -- images/sec of GANsformer synthesis (BASELINE.json configs, default configs[1]: 256x256, K=16, batch 32/GPU)
 + attention roofline.
 
-    python bench.py [--gpus N] [--steps K] [--warmup W] [--impl ours|reference] [--config 1|2|3|5]
+    python bench.py [--gpus N] [--steps K] [--warmup W] [--impl ours|reference] [--config 1|2|3|5] [--dump-outputs DIR]
     python -m torch.distributed.run --nnodes=1 --nproc-per-node N --master-addr 127.0.0.1 --master-port P bench.py --gpus N ...
 
 A "step" is one generator forward over one batch of synthetic latents (weak scaling: every rank runs its own slice of a
@@ -20,6 +20,11 @@ globally seeded batch, no data-path collective -- SURVEY 8e).  Rank 0 prints ONE
   roofline_duplex  BASELINE's second named metric: the 12 duplex layer calls of configs[2] (K=32, batch 64), same formula
   train_step       BASELINE configs[3]: G+D training step, data-parallel with the NCCL gradient all-reduce, at every N
   cpu_baseline     the CPU oracle (oracle/generator.py, fp32, pinned thread count, median of 3) on a bounded sample, N = 1 only
+
+--dump-outputs DIR writes DIR/images.npy: the float32 images [B, 3, R, R] the last timed step returned (rank 0's slice).
+Weights (seed 0) and latents (seed 1) are fixed, so two builds run with the same arguments can be compared image for image.
+The comparison needs a tolerance: cuDNN picks its TF32 algorithms per process, and two runs of one build differed by
+2.6e-4 relative RMS (NVIDIA B200, 1000 W power limit).
 
 --impl reference times the reference arm: the reference's own implementation cannot be installed (no source in
 /root/reference, TensorFlow 1.14 unavailable -- DESIGN.md), so per the tier contract the arm is the CPU oracle port.
@@ -69,6 +74,21 @@ def measured_peak_gbs():
             return float(json.load(f)["hbm_gbs"]), "measured (MEASURED_PEAKS.json, burst copy)"
     except Exception:
         return 6650.0, "fallback (B200_PROFILING.md)"
+
+
+DUMP_LIMIT_BYTES = 64 << 20
+
+
+def dump_outputs(out_dir: str, arrays: dict) -> None:
+    """Writes each array as out_dir/<name>.npy (float32)."""
+    import numpy as np
+    arrays = {n: a.detach().float().cpu().numpy() for n, a in arrays.items()}
+    total = sum(a.nbytes for a in arrays.values())
+    if total > DUMP_LIMIT_BYTES:
+        raise RuntimeError(f"--dump-outputs: {total} bytes exceed the {DUMP_LIMIT_BYTES} byte limit")
+    os.makedirs(out_dir, exist_ok=True)
+    for name, a in arrays.items():
+        np.save(os.path.join(out_dir, name + ".npy"), a)
 
 
 def conv_roofline_probe(device, iters: int = 5):
@@ -352,9 +372,9 @@ def train_probe(device, rank, world, steps: int = 3, warmup: int = 1, B: int = 3
 
 
 def run_reference(args):
-    """The reference arm: the reference's own implementation cannot be installed or run (no source under /root/reference,
-    TensorFlow 1.14 unavailable), so per the tier contract this times the CPU oracle port on the host cores: pinned thread
-    count, median of >= 3 steps of a bounded sample (2 images per step; config 1: its exact batch of 4)."""
+    """The reference arm: the reference's own implementation cannot be installed or run (its source is not available and
+    it needs TensorFlow 1.14), so this times the CPU oracle port on the host cores: pinned thread count, median of --steps
+    steps of a bounded sample (2 images per step; config 1: its exact batch of 4)."""
     rank = int(os.environ.get("RANK", 0))
     if rank != 0:
         return 0
@@ -363,7 +383,7 @@ def run_reference(args):
     import gansformer_b200 as gf
     G = gf.Generator(resolution=RES, components_num=K_LATENTS, latent_dim=LATENT_DIM, kmeans=DUPLEX)
     sample_b = B_PER_GPU if args.config == 1 else (1 if RES >= 512 else 2)
-    steps, warmup = max(3, min(args.steps, 5)), 1
+    steps, warmup = args.steps, 1
     ips, t, cores = cpu_oracle_run(G.state_dict(), steps, warmup, sample_b)
     line = {"impl": "reference", "metric": METRIC, "value": ips, "unit": UNIT, "n_gpus": args.gpus, "steps": steps, "warmup": warmup,
             "ms_per_step": t * 1e3, "higher_is_better": True, "scaling": "weak", "vs_baseline": None, "dtype": "f32", "data": "synthetic",
@@ -484,10 +504,12 @@ def run_ours(args):
     torch.cuda.profiler.start()              # ncu --profile-from-start off captures exactly the timed steps
     ev0.record()
     for _ in range(args.steps):
-        step_resident()
+        img = step_resident()
     ev1.record()
     torch.cuda.synchronize()
     torch.cuda.profiler.stop()
+    if args.dump_outputs and rank == 0:              # before the next replay overwrites the graph's static output
+        dump_outputs(args.dump_outputs, {"images": img})
     dist_mod.barrier()
     clocks = sampler.stop() if rank == 0 else None
     t_total = dist_mod.max_over_ranks(ev0.elapsed_time(ev1) * 1e-3, device)
@@ -673,7 +695,12 @@ def main():
     ap.add_argument("--no-train-probe", action="store_true", help="skip the BASELINE configs[3] probe (G+D training step, train_step object)")
     ap.add_argument("--train-probe", action="store_true", help="(kept for compatibility: the probe now runs at every N by default)")
     ap.add_argument("--train-timeout", type=float, default=240.0, help="watchdog of the training probe in seconds")
+    ap.add_argument("--dump-outputs", metavar="DIR", help="write the images of the last timed step to DIR/images.npy (--impl ours)")
     args = ap.parse_args()
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
+    if args.dump_outputs and args.impl != "ours":
+        ap.error("--dump-outputs applies to --impl ours")
     if args.impl == "ours":
         args.warmup = max(args.warmup, 3)
     rc = run_reference(args) if args.impl == "reference" else run_ours(args)

@@ -2,6 +2,8 @@
 
 PARITY UNPINNED: the reference ships no fixtures for this path (no source at all, SURVEY.md section 0), so these
 vectors pin the *oracle*, and through it the CUDA kernels, against silent drift -- not against the reference.
+Attention probabilities and centroids are stored whole; of each layer output only the fixed sample ``out_sample``
+is stored, which keeps the file small (the tests compare the full output with the live fp64 oracle).
 Run from the repo root:  python tests/golden/make_golden.py
 """
 import itertools
@@ -16,6 +18,12 @@ sys.path.insert(0, ROOT)
 from oracle import bipartite as ob  # noqa: E402
 
 B, C, H, W, D, P = 2, 64, 8, 16, 16, 16
+OUT_STRIDE = 5          # coprime with C and W: the sample covers every channel and every pixel column
+
+
+def out_sample(out_nhwc):
+    """The stored sample of a channels-last layer output (numpy array or tensor): every OUT_STRIDE-th element."""
+    return out_nhwc.reshape(-1)[::OUT_STRIDE]
 
 
 def cases():
@@ -63,7 +71,7 @@ def main():
                                              use_pos=c["use_pos"], return_att=True, kmeans_iters=c.get("kmeans_iters", 1),
                                              img2ltnt=bool(c.get("img2ltnt")), num_heads=c.get("num_heads", 1))
         name = case_name(c)
-        store[name + "/out"] = out.permute(0, 2, 3, 1).contiguous().numpy().astype(np.float32)   # channels-last
+        store[name + "/out_sample"] = out_sample(out.permute(0, 2, 3, 1).contiguous().numpy()).astype(np.float32)   # channels-last
         store[name + "/att"] = att.numpy().astype(np.float32)
         if cen is not None:
             store[name + "/cen"] = cen.numpy().astype(np.float32)

@@ -98,7 +98,12 @@ def test_layer_matches_golden(gf, cuda_dev, idx, exact):
                                     num_heads=c.get("num_heads", 1))
     if exact:
         assert path == "simt_fp32"
-    check_close(out, torch.from_numpy(gold[name + "/out"]), path, name + "/out", tol_scale=1.5 if c.get("kmeans_iters", 1) > 1 else 1.0)
+    # the full output against the fp64 oracle, which the stored sample pins
+    ref, _, _ = ob.transformer_layer(x, y, w, integration=c["integration"], norm=norm, duplex=c["duplex"], use_pos=c["use_pos"],
+                                     kmeans_iters=c.get("kmeans_iters", 1), img2ltnt=bool(c.get("img2ltnt")), num_heads=c.get("num_heads", 1))
+    ref = ref.permute(0, 2, 3, 1).contiguous()
+    np.testing.assert_allclose(mg.out_sample(ref.numpy()), gold[name + "/out_sample"], rtol=2e-6, atol=2e-6)
+    check_close(out, ref, path, name + "/out", tol_scale=1.5 if c.get("kmeans_iters", 1) > 1 else 1.0)
     a_atol = 1e-6 if path == "simt_fp32" else 2e-3
     assert (att.cpu().double() - torch.from_numpy(gold[name + "/att"]).double()).abs().max() <= a_atol + (1e-4 if exact else 5e-3)
     if c["duplex"]:

@@ -424,6 +424,7 @@ def test_bench_reference_arm_json_contract():
     for key in ("metric", "value", "n_gpus", "steps", "warmup", "ms_per_step", "scaling", "vs_baseline", "dtype", "data", "config",
                 "e2e", "cpu_baseline"):
         assert key in line, key
+    assert line["steps"] == 1
     assert line["value"] > 0 and line["cpu_baseline"]["kind"] == "port" and line["cpu_baseline"]["cores"] >= 1
     assert line["e2e"]["h2d_bytes_per_step"] == 0 and line["e2e"]["d2h_bytes_per_step"] == 0
     assert "workload" in line["config"] and "model" not in line["config"]
