@@ -30,7 +30,8 @@ EXPORTS = ("gf_attn_abi_version", "gf_last_error", "gf_attn_last_path", "gf_attn
            "gf_attn_fold_weights", "gf_attn_workspace_bytes", "gf_attn_prologue", "gf_attn_simplex_fwd",
            "gf_attn_duplex_fwd", "gf_attn_norm_stats", "gf_attn_launch_count",
            "gf_attn_simplex_fwd_ex", "gf_attn_duplex_fwd_ex", "gf_attn_prologue_ex", "gf_attn_simplex_bwd", "gf_attn_last_centroid_path", "gf_attn_debug_layout",
-           "gf_attn_prologue_batch", "gf_attn_tc_eligible", "gf_attn_simplex_bwd_ex", "gf_attn_dropout_mask")
+           "gf_attn_prologue_batch", "gf_attn_tc_eligible", "gf_attn_simplex_bwd_ex", "gf_attn_dropout_mask",
+           "gf_attn_centroid_recompute", "gf_attn_centroid_bwd")
 # include/gf_ops.h
 OPS_EXPORTS = ("gf_chan_scale_nhwc", "gf_blur_up_nhwc", "gf_upsample2x_nchw", "gf_bias_act_nhwc", "gf_demod_coef", "gf_torgb_nhwc", "gf_fir4_nhwc", "gf_blur_up_phases_nhwc", "gf_torgb_scale_nhwc", "gf_mapping_fwd", "gf_conv3x3_pack_weights", "gf_conv3x3_nhwc_tf32", "gf_demod_coef_batch")
 
@@ -90,6 +91,8 @@ def load() -> ctypes.CDLL:
     lib.gf_attn_prologue_batch.argtypes = [c_int, c_void_p, c_void_p, c_void_p, c_void_p, c_void_p, c_void_p]
     lib.gf_attn_simplex_bwd.argtypes = [POINTER(GfAttnDesc)] + [c_void_p] * 11
     lib.gf_attn_simplex_bwd_ex.argtypes = [POINTER(GfAttnDesc)] + [c_void_p] * 10 + [ctypes.c_float, ctypes.c_uint32, c_void_p, c_void_p, c_void_p]
+    lib.gf_attn_centroid_recompute.argtypes = [POINTER(GfAttnDesc)] + [c_void_p] * 8
+    lib.gf_attn_centroid_bwd.argtypes = [POINTER(GfAttnDesc)] + [c_void_p] * 10
     lib.gf_attn_dropout_mask.argtypes = [POINTER(GfAttnDesc), ctypes.c_float, ctypes.c_uint32, c_void_p, c_void_p, c_void_p]
     lib.gf_chan_scale_nhwc.argtypes = [c_void_p, c_void_p, c_int, c_void_p, c_int, c_int, c_int, c_void_p]
     lib.gf_blur_up_nhwc.argtypes = [c_void_p, c_void_p, c_void_p, c_int, c_int, c_int, c_int, ctypes.c_float, c_void_p]

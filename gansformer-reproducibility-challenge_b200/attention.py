@@ -381,7 +381,8 @@ class BipartiteAttention(nn.Module):
         self.num_heads, self.integration, self.norm = num_heads, integration, norm
         self.duplex, self.use_pos, self.exact_fp32 = bool(kmeans), use_pos, exact_fp32
         self.kmeans_iters, self.img2ltnt, self.iterative = int(kmeans_iters), bool(img2ltnt), bool(iterative and kmeans)
-        self.att_dp = float(att_dp)                       # attention dropout, active in training mode only (reference: p ~ 0.12)
+        self.att_dp = float(att_dp)                       # attention dropout, active in training mode only (reference: p ~ 0.12);
+        # duplex layers drop pass B's probabilities (over the latents) only, never pass A's softmax over the grid cells
         _DP_SALT[0] += 1
         self.dp_salt = _DP_SALT[0] * 0x9E3779B1 & 0xFFFFFFFF   # distinct masks per layer
         for name, shape in param_shapes(dim, latent_dim, components_num, self.pos_dim, integration, self.duplex, self.kmeans_iters, self.img2ltnt,
@@ -407,16 +408,21 @@ class BipartiteAttention(nn.Module):
         if torch.is_grad_enabled() and (x.requires_grad or y.requires_grad or any(p.requires_grad for p in self.parameters())):
             if postop is not None:
                 raise RuntimeError("the fused post-op is inference-only; apply noise/bias/activation outside when training")
-            if self.att_dp > 0.0 and self.training and (self.duplex or self.num_heads != 1):
-                raise NotImplementedError("attention dropout is implemented for single-head simplex layers")
+            if self.att_dp > 0.0 and self.training:
+                if self.num_heads != 1:
+                    raise NotImplementedError("attention dropout needs a single-head layer: the multi-head backward (torch composite) "
+                                              "cannot apply the dropout mask")
+                if self.duplex and self.norm not in ("layer", None, "none"):
+                    raise NotImplementedError("attention dropout on a duplex layer needs norm 'layer' or None: there is no backward "
+                                              "kernel for instance / batch norm")
             if centroids_init is not None:
                 raise RuntimeError("iterative centroid carry (centroids_init) is an inference feature in this build")
             from .autograd import bipartite_attention_autograd
             return bipartite_attention_autograd(self, x, y, centroids, return_att)
         dp = self.dropout_postop(x.device)
         if dp:
-            if self.duplex or self.num_heads != 1:
-                raise NotImplementedError("attention dropout is implemented for single-head simplex layers")
+            if self.num_heads != 1:
+                raise NotImplementedError("attention dropout needs a single-head layer (one mask column per latent)")
             postop = {**(postop or {"act": "linear", "gain": 1.0}), **dp}
         return bipartite_attention_forward(x, y, self.param_dict(), self._plan, integration=self.integration,
                                            norm=self.norm, duplex=self.kmeans_iters if self.duplex else 0, num_heads=self.num_heads,

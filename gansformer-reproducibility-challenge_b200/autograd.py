@@ -3,8 +3,11 @@
 Forward = the C-ABI CUDA kernels.  Backward of a simplex layer with layer norm (or none): the hand-written stage-T
 backward kernel ``gf_attn_simplex_bwd`` (activation gradient + the per-token gradients of logits / control signal), two
 batched GEMMs for the reductions over tokens, and torch autograd through the tiny per-image tables of stages W and I
-(``folded_tables``).  Everything else (duplex, instance / batch norm, CPU tensors): PyTorch autograd through a
-recomputation of the direct-form algebra with torch ops (``composite_forward``).
+(``folded_tables``).  A duplex layer trained with attention dropout takes the same route for stage T; its pass A (the
+centroid softmax over the grid cells) is recomputed and differentiated by ``gf_attn_centroid_recompute`` /
+``gf_attn_centroid_bwd`` (``_PassA``), with torch autograd through the [B, k, *] tables around it (``duplex_queries`` /
+``duplex_query_tables``).  Everything else (plain duplex layers, instance / batch norm, multi-head layers, CPU tensors):
+PyTorch autograd through a recomputation of the direct-form algebra with torch ops (``composite_forward``).
 """
 from __future__ import annotations
 
@@ -92,10 +95,11 @@ def composite_forward(x, y, p, *, integration, norm, duplex, use_pos, centroids=
     return out.reshape(B, H, W, C), cen
 
 
-def folded_tables(y, p, *, H, W, C, integration, use_pos):
+def folded_tables(y, p, *, H, W, C, integration, use_pos, cen=None, img2ltnt=False):
     """Stages W + I in differentiable torch ops: (latents y [B,k,D], raw parameters) -> the per-image tables stage T and its
     backward consume, in the workspace layout: Kp [B,KP,C], Vt [B,Cout,KP], Rt [B,H,KP] (-inf in the padded latents),
-    Ct [B,W,KP].  Same algebra as csrc/gf_fold.cu (simplex)."""
+    Ct [B,W,KP].  Same algebra as csrc/gf_fold.cu.  Duplex layers: cen [B,k,C] = the centroids, keys from them through wkc;
+    img2ltnt: values from the latents modulated by the centroids."""
     B, k, _ = y.shape
     KP = 16 if k <= 16 else 32
     s = 1.0 / math.sqrt(C)
@@ -108,7 +112,13 @@ def folded_tables(y, p, *, H, W, C, integration, use_pos):
     kconst = p["bk"][None, :].expand(k, C)
     if use_pos:
         kconst = kconst + p["pos_latent"] @ _e(p["wpk"])
-    kp_all = y @ (_e(p["wk"]) @ qfold) + (kconst @ qfold)[None]          # [B, k, C + pd + 1]
+    if cen is None:
+        kp_all = y @ (_e(p["wk"]) @ qfold) + (kconst @ qfold)[None]      # [B, k, C + pd + 1]
+    else:
+        kp_all = cen @ (_e(p["wkc"]) @ qfold) + (kconst @ qfold)[None]
+    if img2ltnt:
+        ym = y.mean(dim=2, keepdim=True)
+        y = (y - ym) * torch.rsqrt(((y - ym) ** 2).mean(dim=2, keepdim=True) + 1e-8) * (1.0 + cen @ _e(p["wi2l"]) + p["bi2l"])
     Kp = torch.nn.functional.pad(kp_all[:, :, :C], (0, 0, 0, KP - k))
     kap0 = kp_all[:, :, C + pd]
     if use_pos:
@@ -131,8 +141,85 @@ def folded_tables(y, p, *, H, W, C, integration, use_pos):
     return Kp.contiguous(), Vt.contiguous(), Rt.contiguous(), Ct.contiguous(), cb.contiguous()
 
 
-def _kernel_backward_ok(m, x) -> bool:
-    return (not m.duplex) and m.norm in ("layer", None, "none") and m.num_heads == 1 and x.is_cuda and x.dtype == torch.float32
+def duplex_queries(src, p, *, first, use_pos):
+    """Pass-A queries Qy [B,k,C] of one k-means iteration: from the latents (first iteration) or the previous centroids (wcq)."""
+    qy = src @ _e(p["wq2"] if first else p["wcq"]) + p["bq2"]
+    if use_pos:
+        qy = qy + (p["pos_latent"] @ _e(p["wpq2"]))[None]
+    return qy
+
+
+def duplex_query_tables(qy, p, *, H, W, C, use_pos):
+    """Pass-A tables in the workspace layout from the queries: Sa[j,t] = x_t.M[j] + Rt2[h,j] + Ct2[w,j] = Qy_j.Kx_t / sqrt(C),
+    Kx = X wk2 + bk2 (+ the grid positional term through wpk2).  M [B,KP,C] (zero rows in the padded latents), Rt2 [B,H,KP]
+    (-inf there), Ct2 [B,W,KP].  The bk2 term is constant over the tokens (the forward's fold drops it); it rides in Rt2 so the
+    tables reproduce the direct form's scores."""
+    B, k, _ = qy.shape
+    KP = 16 if k <= 16 else 32
+    s = 1.0 / math.sqrt(C)
+    M = torch.nn.functional.pad((qy @ _e(p["wk2"]).t()) * s, (0, 0, 0, KP - k))
+    kap0 = (qy @ p["bk2"]) * s                                           # [B, k]
+    if use_pos:
+        half = p["pos_latent"].shape[1] // 2
+        qp = (qy @ _e(p["wpk2"]).t()) * s                                # [B, k, pd]
+        row, col = _axis(H, half, qy.device).to(qy.dtype), _axis(W, half, qy.device).to(qy.dtype)
+        rt = torch.einsum("hp,bjp->bhj", row, qp[:, :, :half]) + kap0[:, None, :]
+        ct = torch.einsum("wp,bjp->bwj", col, qp[:, :, half:])
+    else:
+        rt = kap0[:, None, :].expand(B, H, k)
+        ct = torch.zeros(B, W, k, device=qy.device, dtype=qy.dtype)
+    Rt2 = torch.cat([rt, torch.full((B, H, KP - k), -math.inf, device=qy.device, dtype=qy.dtype)], dim=2) if KP > k else rt
+    Ct2 = torch.nn.functional.pad(ct, (0, KP - k))
+    return M.contiguous(), Rt2.contiguous(), Ct2.contiguous()
+
+
+class _PassA(torch.autograd.Function):
+    """Xbar [B,k,C] = softmax over the tokens of (X M^T + Rt2 + Ct2), times X: duplex pass A recomputed in fp32 by
+    gf_attn_centroid_recompute.  Backward: gf_attn_centroid_bwd, which adds the activation gradient of pass A into `dx_acc` in
+    place (the stage-T gradient, written before autograd reaches this node) instead of returning it; the reductions over the
+    tokens are batched GEMMs / sums."""
+
+    @staticmethod
+    def forward(ctx, desc, X, dx_acc, M, Rt2, Ct2):
+        import ctypes
+        from . import _lib
+        B, n, C = X.shape
+        k = desc.k
+        Xbar = torch.empty((B, k, C), dtype=torch.float32, device=X.device)
+        lse = torch.empty((B, k), dtype=torch.float32, device=X.device)
+        ws = torch.empty(_lib.workspace_bytes(desc), dtype=torch.uint8, device=X.device)
+        with torch.cuda.device(X.device):
+            stream = ctypes.c_void_p(torch.cuda.current_stream(X.device).cuda_stream)
+            _lib.check(_lib.load().gf_attn_centroid_recompute(ctypes.byref(desc), X.data_ptr(), M.data_ptr(), Rt2.data_ptr(), Ct2.data_ptr(),
+                                                              Xbar.data_ptr(), lse.data_ptr(), ws.data_ptr(), stream), "gf_attn_centroid_recompute")
+        ctx.desc, ctx.dx_acc = desc, dx_acc
+        ctx.save_for_backward(X, M, Rt2, Ct2, lse, Xbar)
+        return Xbar
+
+    @staticmethod
+    def backward(ctx, dXbar):
+        import ctypes
+        from . import _lib
+        X, M, Rt2, Ct2, lse, Xbar = ctx.saved_tensors
+        d = ctx.desc
+        B, n, C = X.shape
+        KP = M.shape[1]
+        dXbar = dXbar.contiguous()
+        dSa = torch.empty((B, n, KP), dtype=torch.float32, device=X.device)
+        with torch.cuda.device(X.device):
+            stream = ctypes.c_void_p(torch.cuda.current_stream(X.device).cuda_stream)
+            _lib.check(_lib.load().gf_attn_centroid_bwd(ctypes.byref(d), X.data_ptr(), M.data_ptr(), Rt2.data_ptr(), Ct2.data_ptr(), lse.data_ptr(),
+                                                        Xbar.data_ptr(), dXbar.data_ptr(), ctx.dx_acc.data_ptr(), dSa.data_ptr(), stream),
+                       "gf_attn_centroid_bwd")
+        dM = torch.bmm(dSa.transpose(1, 2), X)                           # [B, KP, C]
+        dS4 = dSa.view(B, d.H, d.W, KP)
+        return None, None, None, dM, dS4.sum(dim=2), dS4.sum(dim=1)
+
+
+def _kernel_backward_ok(m, x, dropout=None) -> bool:
+    """Simplex layers, and duplex layers trained with attention dropout (plain duplex layers keep the composite)."""
+    return ((not m.duplex) or bool(dropout)) and m.norm in ("layer", None, "none") and m.num_heads == 1 and x.is_cuda \
+        and x.dtype == torch.float32
 
 
 class _FusedAttention(torch.autograd.Function):
@@ -156,8 +243,8 @@ class _FusedAttention(torch.autograd.Function):
     def backward(ctx, g_out, g_att, g_cen):
         m = ctx.module
         x, y, *params = ctx.saved_tensors
-        if _kernel_backward_ok(m, x):
-            return (None, None, None, None, *_kernel_backward(m, ctx.names, x, y, params, g_out, ctx.dropout))
+        if _kernel_backward_ok(m, x, ctx.dropout):
+            return (None, None, None, None, *_kernel_backward(m, ctx.names, x, y, params, g_out, ctx.dropout, ctx.centroids))
         if ctx.dropout:
             raise NotImplementedError("attention dropout needs the stage-T backward kernel (single-head simplex, layer norm / none)")
         with torch.enable_grad():
@@ -171,19 +258,33 @@ class _FusedAttention(torch.autograd.Function):
         return (None, None, None, None, *grads)
 
 
-def _kernel_backward(m, names, x, y, params, g_out, dropout=None):
-    """d(loss)/d(x, y, params) of a simplex layer through gf_attn_simplex_bwd (see the module docstring)."""
+def _kernel_backward(m, names, x, y, params, g_out, dropout=None, centroids=None):
+    """d(loss)/d(x, y, params) through gf_attn_simplex_bwd (stage T) and, for a duplex layer, _PassA (see the module docstring)."""
     import ctypes
     from . import _lib
     B, H, W, C = x.shape
     n, k = H * W, y.shape[1]
+    xc, gc = x.detach().contiguous(), g_out.detach().contiguous()
+    dX = torch.empty_like(xc)                    # stage T writes it; pass A's backward adds its part in place
     with torch.enable_grad():
         ys = y.detach().requires_grad_(True)
         ps = [p.detach().requires_grad_(True) for p in params]
-        Kp, Vt, Rt, Ct, cb = folded_tables(ys, dict(zip(names, ps)), H=H, W=W, C=C, integration=m.integration, use_pos=m.use_pos)
+        pd = dict(zip(names, ps))
+        cen = None
+        if m.duplex:
+            if centroids is not None:            # given centroids: no pass A to differentiate
+                cen = centroids.detach()
+            else:
+                desc_a = _lib.make_desc(B, H, W, C, k, y.shape[2], heads=1, norm=m.norm, integration=m.integration,
+                                        pos_dim=m.pos_dim if m.use_pos else 0, duplex=1, flags=0)
+                X = xc.reshape(B, n, C)
+                for it in range(m.kmeans_iters):
+                    qy = duplex_queries(ys if it == 0 else cen, pd, first=it == 0, use_pos=m.use_pos)
+                    M, Rt2, Ct2 = duplex_query_tables(qy, pd, H=H, W=W, C=C, use_pos=m.use_pos)
+                    cen = _PassA.apply(desc_a, X, dX, M, Rt2, Ct2) @ _e(pd["wv2"]) + pd["bv2"]
+        Kp, Vt, Rt, Ct, cb = folded_tables(ys, pd, H=H, W=W, C=C, integration=m.integration, use_pos=m.use_pos, cen=cen,
+                                           img2ltnt=bool(m.duplex and m.img2ltnt))
     KP, Cout = Kp.shape[1], Vt.shape[1]
-    xc, gc = x.detach().contiguous(), g_out.detach().contiguous()
-    dX = torch.empty_like(xc)
     dS = torch.empty((B, n, KP), dtype=torch.float32, device=x.device)
     P = torch.empty_like(dS)
     dCtl = torch.empty((B, n, Cout), dtype=torch.float32, device=x.device)

@@ -12,6 +12,15 @@
 //     dK'[b] = dS[b]^T X[b],   dV^T[b] = dCtl[b]^T P[b],   dRt = sum_w dS,   dCt = sum_h dS,
 // and the chain rule through stages I and W is torch autograd over tiny [B,k,*] tensors.
 // Replaces ~45 full passes over [B,n,C]-sized tensors of the direct-form autograd composite by 8.
+//
+// Backward of duplex pass A (the centroid softmax over the n grid cells), per image, latent j < k, token t:
+//     Sa[j,t] = x_t.M_j + Rt2[h(t),j] + Ct2[w(t),j],   A = softmax_t(Sa),   Xbar = A X.
+// gf_attn_centroid_recompute re-runs the pass-A kernel of gf_simt.cu on the caller's fp32 tables (Xbar and lse_j =
+// log sum_t exp Sa[j,t]); centroid_bwd_kernel then, given dXbar, streams the tokens once more (thread = token, two sweeps over
+// the 32-channel chunks):
+//     A[j,t] = exp(Sa - lse_j),  dA = x_t.dXbar_j,  r_j = Xbar_j.dXbar_j,  dSa = A (dA - r),
+//     dX += dSa.M + A.dXbar   (accumulated onto the stage-T activation gradient: no extra full-size pass)
+// and writes dSa [B,n,KP]; the caller reduces dM = dSa^T X, dRt2 = sum_w dSa, dCt2 = sum_h dSa.
 #include <string.h>
 #include "gf_common.cuh"
 
@@ -252,9 +261,162 @@ __global__ void __launch_bounds__(BTM) token_bwd_kernel(const BwdParams P) {
   }
 }
 
+struct CenBwdParams {
+  const float* X; const float* M; const float* Rt; const float* Ct; const float* lse; const float* Xbar; const float* dXbar;
+  float* dX; float* dSa;
+  int n, H, W, C, k;
+};
+
+// M / dXbar chunk [KP][32] of image b; rows j >= k are zero, so the padded latents contribute exactly nothing
+template <int KP>
+__device__ __forceinline__ void cen_load_tables(float (*ms)[BCH], float (*gs)[BCH], const float* __restrict__ Mb, const float* __restrict__ Gb,
+                                                int k, int C, int c0) {
+  for (int i = threadIdx.x; i < KP * BCH / 4; i += BTM) {
+    const int j = i / (BCH / 4), c4 = (i % (BCH / 4)) * 4;
+    float4 m = make_float4(0.f, 0.f, 0.f, 0.f), g = m;
+    if (j < k) {
+      m = __ldg(reinterpret_cast<const float4*>(Mb + (size_t)j * C + c0 + c4));
+      g = __ldg(reinterpret_cast<const float4*>(Gb + (size_t)j * C + c0 + c4));
+    }
+    *reinterpret_cast<float4*>(&ms[j][c4]) = m;
+    *reinterpret_cast<float4*>(&gs[j][c4]) = g;
+  }
+}
+
+template <int KP>
+__global__ void __launch_bounds__(BTM) centroid_bwd_kernel(const CenBwdParams P) {
+  __shared__ __align__(16) float xs[BTM][BXS];     // x chunk (sweep 1), dX chunk (sweep 2)
+  __shared__ __align__(16) float ms[KP][BCH];      // M chunk
+  __shared__ __align__(16) float gs[KP][BCH];      // dXbar chunk
+  __shared__ float rs[KP];                         // r_j = Xbar_j . dXbar_j of this image
+
+  const int b = blockIdx.y, t0 = blockIdx.x * BTM, tid = threadIdx.x, t = t0 + tid;
+  const int n = P.n, C = P.C, k = P.k;
+  const bool valid = t < n;
+  const float* Xb = P.X + (size_t)b * n * C;
+  const float* Mb = P.M + (size_t)b * KP * C;
+  const float* Gb = P.dXbar + (size_t)b * k * C;
+  const float* XBb = P.Xbar + (size_t)b * k * C;
+  float* dXb = P.dX + (size_t)b * n * C;
+
+  float s[KP], da[KP];
+  {
+    const int h = valid ? t / P.W : 0, w = valid ? t % P.W : 0;
+    const float* rt = P.Rt + ((size_t)b * P.H + h) * KP;
+    const float* ct = P.Ct + ((size_t)b * P.W + w) * KP;
+#pragma unroll
+    for (int j = 0; j < KP; ++j) { s[j] = rt[j] + ct[j]; da[j] = 0.f; }
+  }
+  float racc = 0.f;                                // thread j < k: its latent's r_j, chunk by chunk
+  // ---- sweep 1: logits Sa and dA = x.dXbar
+  for (int c0 = 0; c0 < C; c0 += BCH) {
+    __syncthreads();
+    bwd_load_chunk(xs, Xb, t0, n, C, c0);
+    cen_load_tables<KP>(ms, gs, Mb, Gb, k, C, c0);
+    __syncthreads();
+    if (tid < k) {
+#pragma unroll
+      for (int c4 = 0; c4 < BCH; c4 += 4) {
+        const float4 xb = __ldg(reinterpret_cast<const float4*>(XBb + (size_t)tid * C + c0 + c4));
+        const float4 g = *reinterpret_cast<const float4*>(&gs[tid][c4]);
+        racc = fmaf(xb.x, g.x, fmaf(xb.y, g.y, fmaf(xb.z, g.z, fmaf(xb.w, g.w, racc))));
+      }
+    }
+#pragma unroll
+    for (int c4 = 0; c4 < BCH; c4 += 4) {
+      const float4 x = *reinterpret_cast<const float4*>(&xs[tid][c4]);
+#pragma unroll
+      for (int j = 0; j < KP; ++j) {
+        const float4 m = *reinterpret_cast<const float4*>(&ms[j][c4]);
+        const float4 g = *reinterpret_cast<const float4*>(&gs[j][c4]);
+        s[j] = fmaf(x.x, m.x, fmaf(x.y, m.y, fmaf(x.z, m.z, fmaf(x.w, m.w, s[j]))));
+        da[j] = fmaf(x.x, g.x, fmaf(x.y, g.y, fmaf(x.z, g.z, fmaf(x.w, g.w, da[j]))));
+      }
+    }
+  }
+  if (tid < KP) rs[tid] = tid < k ? racc : 0.f;
+  __syncthreads();
+  // ---- A and dSa (s = A, da = dSa from here on); padded latents: exactly 0
+  const float* lse = P.lse + (size_t)b * k;
+#pragma unroll
+  for (int j = 0; j < KP; ++j) {
+    float a = 0.f, ds = 0.f;
+    if (j < k) {
+      a = expf(s[j] - __ldg(lse + j));
+      ds = a * (da[j] - rs[j]);
+    }
+    s[j] = a; da[j] = ds;
+  }
+  if (valid) {
+    float4* ds4 = reinterpret_cast<float4*>(P.dSa + ((size_t)b * n + t) * KP);
+#pragma unroll
+    for (int j4 = 0; j4 < KP / 4; ++j4) ds4[j4] = make_float4(da[j4 * 4], da[j4 * 4 + 1], da[j4 * 4 + 2], da[j4 * 4 + 3]);
+  }
+  // ---- sweep 2: dX += dSa.M + A.dXbar
+  for (int c0 = 0; c0 < C; c0 += BCH) {
+    __syncthreads();
+    bwd_load_chunk(xs, dXb, t0, n, C, c0);
+    cen_load_tables<KP>(ms, gs, Mb, Gb, k, C, c0);
+    __syncthreads();
+#pragma unroll
+    for (int c4 = 0; c4 < BCH; c4 += 4) {
+      float4 acc = *reinterpret_cast<const float4*>(&xs[tid][c4]);
+#pragma unroll
+      for (int j = 0; j < KP; ++j) {
+        const float4 m = *reinterpret_cast<const float4*>(&ms[j][c4]);
+        const float4 g = *reinterpret_cast<const float4*>(&gs[j][c4]);
+        acc.x = fmaf(da[j], m.x, fmaf(s[j], g.x, acc.x)); acc.y = fmaf(da[j], m.y, fmaf(s[j], g.y, acc.y));
+        acc.z = fmaf(da[j], m.z, fmaf(s[j], g.z, acc.z)); acc.w = fmaf(da[j], m.w, fmaf(s[j], g.w, acc.w));
+      }
+      *reinterpret_cast<float4*>(&xs[tid][c4]) = acc;           // own row only: no hazard with other threads
+    }
+    __syncthreads();
+    bwd_store_chunk(dXb, xs, t0, n, C, c0);
+  }
+}
+
+// shared checks of the two pass-A entry points: a duplex descriptor (its workspace layout has the pass-A partials), grid limits
+static int centroid_entry_layout(const gf_attn_desc* desc, Layout* L, const char* what) {
+  int rc = make_layout(desc, L);
+  if (rc) return rc;
+  if (!L->duplex) { set_error("%s: desc.duplex is 0 (pass A exists in duplex layers only)", what); return GF_ERR_INVALID; }
+  if (L->B > 65535) { set_error("%s: B > 65535", what); return GF_ERR_UNSUPPORTED; }
+  return GF_OK;
+}
+
 }  // namespace gf
 
 using namespace gf;
+
+extern "C" int gf_attn_centroid_recompute(const gf_attn_desc* desc, const float* X, const float* M, const float* Rt2, const float* Ct2,
+                                          float* Xbar, float* lse, void* ws, void* stream) {
+  Layout L;
+  int rc = centroid_entry_layout(desc, &L, "gf_attn_centroid_recompute");
+  if (rc) return rc;
+  if (!X || !M || !Rt2 || !Ct2 || !Xbar || !lse || !ws) { set_error("gf_attn_centroid_recompute: null pointer"); return GF_ERR_INVALID; }
+  if ((rc = check_device())) return rc;
+  cudaStream_t st = (cudaStream_t)stream;
+  if ((rc = centroid_partials_simt(L, X, M, Rt2, Ct2, (float*)ws + L.w_PART, st))) return rc;
+  return centroid_merge(L, (float*)ws, st, nullptr, 0, Xbar, lse);
+}
+
+extern "C" int gf_attn_centroid_bwd(const gf_attn_desc* desc, const float* X, const float* M, const float* Rt2, const float* Ct2,
+                                    const float* lse, const float* Xbar, const float* dXbar, float* dX, float* dSa, void* stream) {
+  Layout L;
+  int rc = centroid_entry_layout(desc, &L, "gf_attn_centroid_bwd");
+  if (rc) return rc;
+  if (!X || !M || !Rt2 || !Ct2 || !lse || !Xbar || !dXbar || !dX || !dSa) { set_error("gf_attn_centroid_bwd: null pointer"); return GF_ERR_INVALID; }
+  if ((rc = check_device())) return rc;
+  CenBwdParams P;
+  P.X = X; P.M = M; P.Rt = Rt2; P.Ct = Ct2; P.lse = lse; P.Xbar = Xbar; P.dXbar = dXbar; P.dX = dX; P.dSa = dSa;
+  P.n = L.n; P.H = L.H; P.W = L.W; P.C = L.C; P.k = L.k;
+  dim3 grid((L.n + BTM - 1) / BTM, L.B);
+  cudaStream_t st = (cudaStream_t)stream;
+  if (L.KP == 16) centroid_bwd_kernel<16><<<grid, BTM, 0, st>>>(P);
+  else centroid_bwd_kernel<32><<<grid, BTM, 0, st>>>(P);
+  GF_LAUNCH_OK();
+  return GF_OK;
+}
 
 extern "C" int gf_attn_simplex_bwd(const gf_attn_desc* desc, const float* X, const float* dOut, const float* Kp, const float* Vt,
                                    const float* Rt, const float* Ct, float* dX, float* dS, float* Pout, float* dCtl, void* stream) {

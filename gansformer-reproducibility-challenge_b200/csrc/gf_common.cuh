@@ -135,8 +135,12 @@ int dropout_args(const gf_attn_postop* post, DropoutArgs* out);
 int norm_stats(const Layout& L, const gf_attn_desc* d, const float* X, float* ws, cudaStream_t st);
 int centroid_pass_simt(const Layout& L, const gf_attn_desc* d, const float* X, float* ws, cudaStream_t st,
                        const float* in_scale = nullptr, int in_scale_ld = 0);
-// Xbar = merge of the split partials (times the load-side scale, when given)
-int centroid_merge(const Layout& L, float* ws, cudaStream_t st, const float* in_scale = nullptr, int in_scale_ld = 0);
+// pass-A partials (per split: acc [KP][C], running max and denominator) of the CUDA-core kernel on the given tables, into `part`
+int centroid_partials_simt(const Layout& L, const float* X, const float* M, const float* Rt, const float* Ct, float* part, cudaStream_t st);
+// Xbar = merge of the split partials in ws (times the load-side scale, when given); into ws + w_XBAR unless `xbar` is given;
+// lse [B,k] (nullable) = log of each latent's softmax denominator
+int centroid_merge(const Layout& L, float* ws, cudaStream_t st, const float* in_scale = nullptr, int in_scale_ld = 0,
+                   float* xbar = nullptr, float* lse = nullptr);
 // tcgen05 duplex pass A (gf_tc_cen.cu): partials into ws (same format as the CUDA-core kernel), then centroid_merge
 bool tc_centroid_supported(const Layout& L, const gf_attn_desc* d);
 // in_scale: only used when the split count is 1 and the kernel writes the normalised Xbar itself (no merge kernel)

@@ -419,7 +419,8 @@ __global__ void __launch_bounds__(256, 4) finalize_kernel(const float* __restric
                                                        float* __restrict__ Kp, float* __restrict__ Vt,
                                                        float* __restrict__ Rt, float* __restrict__ Ct,
                                                        int H, int W, int C, int k, int D, int p, int KP, int Cout, int LDK,
-                                                       int tf32, int npos, const float* __restrict__ in_scale, int in_ld) {
+                                                       int tf32, int npos, const float* __restrict__ in_scale, int in_ld,
+                                                       const float* __restrict__ CB, float* __restrict__ CBout) {
   // grid (B, blocks): the role index is the slow grid dimension so that the longest-running role (V^T) is dispatched first
   const int b = blockIdx.x;
   const float* kp = kpall + (size_t)b * k * LDK;
@@ -465,6 +466,9 @@ __global__ void __launch_bounds__(256, 4) finalize_kernel(const float* __restric
     return;
   }
   if (blk < nvblk + npos) {
+    // batch-independent constant of the control signal, read by stage T when attention dropout is on (duplex layers)
+    if (b == 0 && CBout)
+      for (int i = (blk - nvblk) * blockDim.x + threadIdx.x; i < Cout; i += npos * blockDim.x) CBout[i] = CB[i];
     const int half = p / 2;
     for (int i = (blk - nvblk) * blockDim.x + threadIdx.x; i < (H + W) * KP; i += npos * blockDim.x) {
       const int r = i / KP, j = i % KP;
@@ -737,7 +741,8 @@ int prologue(const Layout& L, const gf_attn_desc* d, const float* Y, const float
   const int nblk = npos + (with_v ? (L.Cout + 255) / 256 : 0) + (L.KP * L.C + 256 * 8 - 1) / (256 * 8);
   finalize_kernel<<<dim3(L.B, nblk), 256, (size_t)L.k * L.D * sizeof(float), st>>>(ws + L.w_KPALL, Y, f + L.f_AV, f + L.f_CV, f + L.f_ROW, f + L.f_COL,
                                                    ws + L.w_Kp, with_v ? ws + L.w_Vt : nullptr, ws + L.w_Rt, ws + L.w_Ct,
-                                                   L.H, L.W, L.C, L.k, L.D, L.p, L.KP, L.Cout, L.LDK, tf32, npos, in_scale, in_scale_ld);
+                                                   L.H, L.W, L.C, L.k, L.D, L.p, L.KP, L.Cout, L.LDK, tf32, npos, in_scale, in_scale_ld,
+                                                   f + L.f_CB, ws + L.w_CB);
   GF_LAUNCH_OK();
   return GF_OK;
 }
@@ -769,7 +774,8 @@ int duplex_tables_from_centroids(const Layout& L, const gf_attn_desc* d, const f
   const int nblk = npos + (L.KP * L.C + 256 * 8 - 1) / (256 * 8);
   finalize_kernel<<<dim3(L.B, nblk), 256, 0, st>>>(ws + L.w_MALL, Y, nullptr, nullptr, f + L.f_ROW, f + L.f_COL,
                                                    ws + L.w_M, nullptr, ws + L.w_Rt2, ws + L.w_Ct2,
-                                                   L.H, L.W, L.C, L.k, L.D, L.p, L.KP, L.Cout, L.LDK, tf32, npos, in_scale, in_scale_ld);
+                                                   L.H, L.W, L.C, L.k, L.D, L.p, L.KP, L.Cout, L.LDK, tf32, npos, in_scale, in_scale_ld,
+                                                   nullptr, nullptr);
   GF_LAUNCH_OK();
   return GF_OK;
 }

@@ -424,9 +424,9 @@ __global__ void __launch_bounds__(TM) centroid_simt_kernel(const CenParams P) {
   (void)k;
 }
 
-// xbar[b,j,c] = sum_sp exp(m_sp - m) acc_sp[j][c] / sum_sp exp(m_sp - m) l_sp
+// xbar[b,j,c] = sum_sp exp(m_sp - m) acc_sp[j][c] / sum_sp exp(m_sp - m) l_sp;  lse[b,j] = m + log(sum_sp exp(m_sp - m) l_sp)
 __global__ void centroid_merge_kernel(const float* __restrict__ part, float* __restrict__ xbar, int B, int k, int KP, int C, int nsplit,
-                                      const float* __restrict__ in_scale, int in_ld) {
+                                      const float* __restrict__ in_scale, int in_ld, float* __restrict__ lse) {
   const int i = blockIdx.x * blockDim.x + threadIdx.x;
   if (i >= B * k * C) return;
   const int c = i % C, j = (i / C) % k, b = i / (C * k);
@@ -442,12 +442,19 @@ __global__ void centroid_merge_kernel(const float* __restrict__ part, float* __r
     den = fmaf(wgt, o[C + 1], den);
   }
   xbar[i] = num / den * (in_scale ? in_scale[(size_t)b * in_ld + c] : 1.f);     // Xbar of x_in = x * d
+  if (lse && c == 0) lse[(size_t)b * k + j] = m + logf(den);
 }
 
 int centroid_pass_simt(const Layout& L, const gf_attn_desc* d, const float* X, float* ws, cudaStream_t st, const float* in_scale, int in_scale_ld) {
   (void)d;
+  int rc = centroid_partials_simt(L, X, ws + L.w_M, ws + L.w_Rt2, ws + L.w_Ct2, ws + L.w_PART, st);
+  if (rc) return rc;
+  return centroid_merge(L, ws, st, in_scale, in_scale_ld);
+}
+
+int centroid_partials_simt(const Layout& L, const float* X, const float* M, const float* Rt, const float* Ct, float* part, cudaStream_t st) {
   CenParams P;
-  P.X = X; P.M = ws + L.w_M; P.Rt = ws + L.w_Rt2; P.Ct = ws + L.w_Ct2; P.part = ws + L.w_PART;
+  P.X = X; P.M = M; P.Rt = Rt; P.Ct = Ct; P.part = part;
   P.n = L.n; P.H = L.H; P.W = L.W; P.C = L.C; P.k = L.k; P.nsplit = L.nsplit_cen;
   const size_t dyn = (size_t)L.KP * L.C * sizeof(float);
   dim3 grid(L.nsplit_cen, L.B);
@@ -459,12 +466,13 @@ int centroid_pass_simt(const Layout& L, const gf_attn_desc* d, const float* X, f
     centroid_simt_kernel<32><<<grid, TM, dyn, st>>>(P);
   }
   GF_LAUNCH_OK();
-  return centroid_merge(L, ws, st, in_scale, in_scale_ld);
+  return GF_OK;
 }
 
-int centroid_merge(const Layout& L, float* ws, cudaStream_t st, const float* in_scale, int in_scale_ld) {
+int centroid_merge(const Layout& L, float* ws, cudaStream_t st, const float* in_scale, int in_scale_ld, float* xbar, float* lse) {
   const int tot = L.B * L.k * L.C;
-  centroid_merge_kernel<<<(tot + 255) / 256, 256, 0, st>>>(ws + L.w_PART, ws + L.w_XBAR, L.B, L.k, L.KP, L.C, L.nsplit_cen, in_scale, in_scale_ld);
+  centroid_merge_kernel<<<(tot + 255) / 256, 256, 0, st>>>(ws + L.w_PART, xbar ? xbar : ws + L.w_XBAR, L.B, L.k, L.KP, L.C, L.nsplit_cen,
+                                                           in_scale, in_scale_ld, lse);
   GF_LAUNCH_OK();
   return GF_OK;
 }

@@ -99,7 +99,9 @@ typedef struct gf_attn_postop {
    * by the seed; dp_state points to DEVICE memory {uint64 seed, uint64 step} read when the kernel runs (bump `step` on the device
    * between training steps: a replayed CUDA graph then draws fresh masks).  Both kernel families serve it with the same mask (the
    * tcgen05 kernel drops the probabilities before they become GEMM2's operand); the attention map output is the probabilities
-   * BEFORE dropout.  att_dp = 0 or dp_state = NULL: off. */
+   * BEFORE dropout.  att_dp = 0 or dp_state = NULL: off.
+   * Duplex layers: only pass B's softmax over the k latents is dropped (same Philox stream, token = b * n + t); pass A's softmax over
+   * the n grid cells, which builds the centroids, never is. */
   float att_dp;
   uint32_t dp_salt;
   const unsigned long long* dp_state;
@@ -197,12 +199,32 @@ int gf_attn_simplex_bwd(const gf_attn_desc* desc, const float* X, const float* d
                         const float* Rt, const float* Ct, float* dX, float* dS, float* P, float* dCtl, void* stream);
 
 /* gf_attn_simplex_bwd with attention dropout: the same (att_dp, dp_salt, dp_state) as the forward call regenerate the mask;
+ * Stage T of a duplex layer is differentiated here too: the kernel consumes the tables only, so the caller passes a descriptor with
+ * duplex = 0 and tables whose keys come from the centroids (and values from the modulated latents with g_img2ltnt);
  * P then receives the probabilities AFTER dropout q (what dVt = dCtl^T P needs), dS the gradient w.r.t. the logits.
  * cb [Cout] = bo (+1 on the gain half): the constants dropout does not scale -- ctl = sum_j q_j (Vt_j - cb) + cb; the caller adds
  * dcb = sum_tokens dCtl * (1 - sum_j q_j) to the gradient of bo.  cb may be NULL when att_dp == 0. */
 int gf_attn_simplex_bwd_ex(const gf_attn_desc* desc, const float* X, const float* dOut, const float* Kp, const float* Vt,
                            const float* Rt, const float* Ct, float* dX, float* dS, float* P, float* dCtl,
                            float att_dp, uint32_t dp_salt, const unsigned long long* dp_state, const float* cb, void* stream);
+
+/* Backward of duplex pass A, part 1 -- recomputes, in fp32 on the CUDA cores, what the forward's pass A computed from the caller's
+ * differentiable tables: per image, latent j < k, token t,
+ *   Sa[j,t] = x_t.M[j] + Rt2[h(t),j] + Ct2[w(t),j],   A = softmax over the n tokens of Sa,   Xbar = A X,
+ * with M [B,KP,C], Rt2 [B,H,KP] (-inf in the padded latents), Ct2 [B,W,KP] in the workspace layout (1/sqrt(C) folded in, KP = 16 for
+ * k <= 16, else 32).  Outputs: Xbar [B,k,C] and lse [B,k] = log sum_t exp Sa[j,t].  desc.duplex >= 1; ws = a workspace of
+ * gf_attn_workspace_bytes(desc) (its pass-A partials are the scratch).  Split partials are merged in a fixed order: deterministic. */
+int gf_attn_centroid_recompute(const gf_attn_desc* desc, const float* X, const float* M, const float* Rt2, const float* Ct2,
+                               float* Xbar, float* lse, void* ws, void* stream);
+
+/* Backward of duplex pass A, part 2 -- given dXbar [B,k,C] and what gf_attn_centroid_recompute returned for the same tables:
+ *   A = exp(Sa - lse),  dA[j,t] = x_t.dXbar[j],  r_j = Xbar[j].dXbar[j],  dSa = A (dA - r),
+ *   dX [B,n,C] += dSa.M + A.dXbar   (accumulated in place: pass the stage-T activation gradient),
+ *   dSa [B,n,KP] written (0 in the padded latents).
+ * The reductions over the tokens that remain are the caller's: dM[b] = dSa[b]^T X[b], dRt2[b,h,:] = sum_w dSa[b,h,w,:],
+ * dCt2[b,w,:] = sum_h dSa[b,h,w,:].  No host synchronisation (capturable in a CUDA graph). */
+int gf_attn_centroid_bwd(const gf_attn_desc* desc, const float* X, const float* M, const float* Rt2, const float* Ct2,
+                         const float* lse, const float* Xbar, const float* dXbar, float* dX, float* dSa, void* stream);
 
 /* The dropout multipliers themselves, mask [B, H*W, KP] (0 or 1 / (1 - att_dp); KP = 16 for k <= 16, else 32; columns of a
  * multi-head layer: head * seg + j): what the fused kernels apply.  For the composite training path and for tests. */

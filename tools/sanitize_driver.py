@@ -76,6 +76,21 @@ if not only or "dropout" in only:
     out.square().mean().backward()
     torch.cuda.synchronize()
     print("dropout fwd/bwd ok", bool(torch.isfinite(x.grad).all()), flush=True)
+# duplex attention dropout: forward on both kernel families (stage T reads the constants the duplex prologue writes), and the backward
+# through the pass-A recompute / backward kernels (KP = 16 and 32, ragged grid, two k-means iterations)
+if not only or "duplex-dropout" in only:
+    for exact, C, H, W, k, iters in ((False, 128, 16, 16, 16, 1), (True, 96, 10, 13, 20, 2)):
+        attn = gf.BipartiteAttention(C, 16, k, pos_dim=16, kmeans=True, kmeans_iters=iters, att_dp=0.2, exact_fp32=exact).to(dev).train()
+        x = torch.randn(2, H, W, C, device=dev, requires_grad=True)
+        y = torch.randn(2, k, 16, device=dev, requires_grad=True)
+        with torch.no_grad():
+            o0, _, _ = attn(x, y)
+        out, _, _ = attn(x, y)
+        out.square().mean().backward()
+        torch.cuda.synchronize()
+        ok = bool(torch.isfinite(x.grad).all()) and torch.equal(o0, out.detach())
+        print(f"duplex-dropout C={C} k={k} iters={iters} path={gf._lib.last_path()} fwd/bwd ok", ok, flush=True)
+        bad += not ok
 # backward kernel
 if not only or "bwd" in only:
     attn = gf.BipartiteAttention(64, 16, 4, pos_dim=16, integration="both").to(dev)
