@@ -33,7 +33,7 @@ EXPORTS = ("gf_attn_abi_version", "gf_last_error", "gf_attn_last_path", "gf_attn
            "gf_attn_prologue_batch", "gf_attn_tc_eligible", "gf_attn_simplex_bwd_ex", "gf_attn_dropout_mask",
            "gf_attn_centroid_recompute", "gf_attn_centroid_bwd")
 # include/gf_ops.h
-OPS_EXPORTS = ("gf_chan_scale_nhwc", "gf_blur_up_nhwc", "gf_upsample2x_nchw", "gf_bias_act_nhwc", "gf_demod_coef", "gf_torgb_nhwc", "gf_fir4_nhwc", "gf_blur_up_phases_nhwc", "gf_torgb_scale_nhwc", "gf_mapping_fwd", "gf_conv3x3_pack_weights", "gf_conv3x3_nhwc_tf32", "gf_demod_coef_batch")
+OPS_EXPORTS = ("gf_chan_scale_nhwc", "gf_blur_up_nhwc", "gf_upsample2x_nchw", "gf_bias_act_nhwc", "gf_demod_coef", "gf_torgb_nhwc", "gf_fir4_nhwc", "gf_blur_up_phases_nhwc", "gf_torgb_scale_nhwc", "gf_mapping_fwd", "gf_conv3x3_pack_weights", "gf_conv3x3_nhwc_tf32", "gf_demod_coef_batch", "gf_conv3x3_nhwc_tf32_ex", "gf_conv3x3_last_variant")
 
 
 class GfAttnDesc(ctypes.Structure):
@@ -108,6 +108,8 @@ def load() -> ctypes.CDLL:
     lib.gf_mapping_fwd.argtypes = [c_void_p, c_void_p, c_void_p, c_void_p, ctypes.c_float, c_void_p, c_int, c_int, c_int, c_int, c_void_p]
     lib.gf_conv3x3_pack_weights.argtypes = [c_void_p, c_void_p, c_int, c_int, ctypes.c_float, c_void_p]
     lib.gf_conv3x3_nhwc_tf32.argtypes = [c_void_p, c_void_p, c_void_p, c_int, c_int, c_int, c_int, c_int, c_void_p]
+    lib.gf_conv3x3_nhwc_tf32_ex.argtypes = [c_void_p, c_void_p, c_void_p] + [c_int] * 8 + [c_void_p]
+    lib.gf_conv3x3_last_variant.argtypes = [POINTER(c_int)] * 3
     lib.gf_demod_coef_batch.argtypes = [c_void_p, c_int, c_int, ctypes.c_float, c_void_p]
     lib.gf_torgb_nhwc.argtypes = [c_void_p, c_void_p, c_void_p, c_int, c_void_p, ctypes.c_float, c_void_p, c_int, c_int, c_int, c_void_p]
     for name in OPS_EXPORTS:
@@ -169,3 +171,10 @@ def last_centroid_path() -> str:
 
 def last_path() -> str:
     return PATH_NAMES.get(load().gf_attn_last_path(), "?")
+
+
+def conv3x3_last_variant() -> tuple:
+    """(version, bn, mt) of the convolution kernel the last gf_conv3x3_nhwc_tf32[_ex] call on this thread launched."""
+    v = (c_int(0), c_int(0), c_int(0))
+    check(load().gf_conv3x3_last_variant(*(byref(i) for i in v)), "gf_conv3x3_last_variant")
+    return tuple(i.value for i in v)

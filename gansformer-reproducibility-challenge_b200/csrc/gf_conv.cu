@@ -473,6 +473,48 @@ static int launch_v2(const float* x, const float* wt, float* y, int B, int H, in
   return GF_OK;
 }
 
+// The twelve instantiations, addressed by (version, BN, MT); NBUF follows from them (one accumulator set only for 256 x 256 tiles)
+typedef int (*LaunchFn)(const float*, const float*, float*, int, int, int, int, int, cudaStream_t);
+struct Variant { int version, bn, mt; LaunchFn fn; };
+static const Variant kVariants[] = {
+    {1, 256, 2, launch<256, 2, 1>},    {1, 256, 1, launch<256, 1, 2>},    {1, 128, 2, launch<128, 2, 2>},
+    {1, 128, 1, launch<128, 1, 2>},    {1, 64, 2, launch<64, 2, 2>},      {1, 64, 1, launch<64, 1, 2>},
+    {2, 256, 2, launch_v2<256, 2, 1>}, {2, 256, 1, launch_v2<256, 1, 2>}, {2, 128, 2, launch_v2<128, 2, 2>},
+    {2, 128, 1, launch_v2<128, 1, 2>}, {2, 64, 2, launch_v2<64, 2, 2>},   {2, 64, 1, launch_v2<64, 1, 2>},
+};
+
+static const Variant* find_variant(int version, int bn, int mt) {
+  for (const Variant& v : kVariants)
+    if (v.version == version && v.bn == bn && v.mt == mt) return &v;
+  return nullptr;
+}
+
+// Dispatch (measured on the generator's shapes, batch 32, tools/conv_bench.py; GF_CONV_V2=0 / 1 and GF_CONV_BIG / GF_CONV_MT force):
+//   * 16 x 16 patches need enough tiles to fill the GPU: fewer than one per SM -> version 1 with 8 x 16 patches (res 16: 0.056 ms,
+//     cuDNN 0.056)
+//   * Cin >= 512 with plenty of tiles -> version 1 with 256 x 256 tiles (res 64: 0.702 ms = 881 TFLOP/s, cuDNN 0.698)
+//   * everything else -> version 2, shared filter-column boxes (res 32: 0.193 ms vs cuDNN 0.199; res 128: 0.721 vs 0.739;
+//     res 256: 0.831 vs 0.781)
+static const Variant* dispatch(int B, int H, int W, int Cin, int Cout) {
+  static const int v2env = []() { const char* e = getenv("GF_CONV_V2"); return e ? atoi(e) : -1; }();
+  const int nsm = num_sms();
+  const long long t2 = H % 16 == 0 ? (long long)B * (H / 16) * (W / 16) * (Cout / (Cout % 256 == 0 ? 256 : (Cout % 128 == 0 ? 128 : 64))) : 0;
+  const bool big_v1 = Cout % 256 == 0 && Cin >= 512 && t2 >= 4ll * nsm;
+  const bool use_v2 = v2env >= 0 ? v2env != 0 : (t2 >= nsm && !big_v1);
+  if (use_v2) {
+    const bool m2 = H % 16 == 0;
+    if (Cout % 256 == 0) return find_variant(2, 256, (m2 && v2env != 2) ? 2 : 1);
+    return find_variant(2, Cout % 128 == 0 ? 128 : 64, m2 ? 2 : 1);
+  }
+  static const int force_mt = []() { const char* e = getenv("GF_CONV_MT"); return e ? atoi(e) : 0; }();     // tuning aid, read once
+  const bool mt2 = (H % 16 == 0) && force_mt != 1 && t2 >= nsm;
+  static const int big_env = []() { const char* e = getenv("GF_CONV_BIG"); return e ? atoi(e) : -1; }();
+  const bool big = big_env >= 0 ? big_env != 0 : big_v1;
+  if (Cout % 256 == 0 && big && H % 16 == 0) return find_variant(1, 256, 2);
+  if (Cout % 256 == 0 && force_mt != 2) return find_variant(1, 256, 1);
+  return find_variant(1, Cout % 128 == 0 ? 128 : 64, mt2 ? 2 : 1);
+}
+
 // w [Cout][Cin][3][3] (PyTorch layout) -> wt [9][Cout][Cin], rounded to the nearest TF32
 __global__ void pack_weights_kernel(const float* __restrict__ w, float* __restrict__ wt, int Cout, int Cin, float scale) {
   const size_t total = (size_t)9 * Cout * Cin;
@@ -499,39 +541,44 @@ extern "C" int gf_conv3x3_pack_weights(const float* w, float* wt, int Cout, int 
   return GF_OK;
 }
 
-extern "C" int gf_conv3x3_nhwc_tf32(const float* x, const float* wt, float* y, int B, int H, int W, int Cin, int Cout, void* stream) {
+static thread_local int g_last_variant[3] = {0, 0, 0};      // (version, bn, mt) the last call on this thread launched, zeros if none
+
+extern "C" int gf_conv3x3_nhwc_tf32_ex(const float* x, const float* wt, float* y, int B, int H, int W, int Cin, int Cout,
+                                       int version, int bn, int mt, void* stream) {
+  g_last_variant[0] = g_last_variant[1] = g_last_variant[2] = 0;
   if (!x || !wt || !y) { set_error("gf_conv3x3_nhwc_tf32: null pointer"); return GF_ERR_INVALID; }
   if (B <= 0 || H % cv::PH || W % cv::PW || Cin % cv::BK || Cout % 64 || Cin <= 0 || Cout <= 0) {
     set_error("gf_conv3x3_nhwc_tf32: needs H %% 8 == 0, W %% 16 == 0, Cin %% 32 == 0, Cout %% 64 == 0 (got B=%d H=%d W=%d Cin=%d Cout=%d)", B, H, W, Cin, Cout);
     return GF_ERR_UNSUPPORTED;
   }
   if (((uintptr_t)x & 15) || ((uintptr_t)wt & 15) || ((uintptr_t)y & 15)) { set_error("gf_conv3x3_nhwc_tf32: pointers must be 16-byte aligned"); return GF_ERR_INVALID; }
+  const cv::Variant* v = nullptr;
+  if (version || bn || mt) {
+    if (!(v = cv::find_variant(version, bn, mt))) {
+      set_error("gf_conv3x3_nhwc_tf32_ex: no instantiation (version=%d, bn=%d, mt=%d): version 1 or 2, bn 64 / 128 / 256, mt 1 or 2, "
+                "or all three 0 for the dispatch", version, bn, mt);
+      return GF_ERR_UNSUPPORTED;
+    }
+    if (Cout % bn || H % (cv::PH * mt)) {
+      set_error("gf_conv3x3_nhwc_tf32_ex: (version=%d, bn=%d, mt=%d) needs Cout %% %d == 0 and H %% %d == 0 (got Cout=%d H=%d)",
+                version, bn, mt, bn, cv::PH * mt, Cout, H);
+      return GF_ERR_UNSUPPORTED;
+    }
+  }
   int rc;
   if ((rc = check_device())) return rc;
-  cudaStream_t st = (cudaStream_t)stream;
-  // Dispatch (measured on the generator's shapes, batch 32, tools/conv_bench.py; GF_CONV_V2=0 / 1 and GF_CONV_BIG / GF_CONV_MT force):
-  //   * 16 x 16 patches need enough tiles to fill the GPU: fewer than one per SM -> version 1 with 8 x 16 patches (res 16: 0.056 ms,
-  //     cuDNN 0.056)
-  //   * Cin >= 512 with plenty of tiles -> version 1 with 256 x 256 tiles (res 64: 0.702 ms = 881 TFLOP/s, cuDNN 0.698)
-  //   * everything else -> version 2, shared filter-column boxes (res 32: 0.193 ms vs cuDNN 0.199; res 128: 0.721 vs 0.739;
-  //     res 256: 0.831 vs 0.781)
-  static const int v2env = []() { const char* e = getenv("GF_CONV_V2"); return e ? atoi(e) : -1; }();
-  const int nsm = num_sms();
-  const long long t2 = H % 16 == 0 ? (long long)B * (H / 16) * (W / 16) * (Cout / (Cout % 256 == 0 ? 256 : (Cout % 128 == 0 ? 128 : 64))) : 0;
-  const bool big_v1 = Cout % 256 == 0 && Cin >= 512 && t2 >= 4ll * nsm;
-  const bool use_v2 = v2env >= 0 ? v2env != 0 : (t2 >= nsm && !big_v1);
-  if (use_v2) {
-    const bool m2 = H % 16 == 0;
-    if (Cout % 256 == 0) return (m2 && v2env != 2) ? cv::launch_v2<256, 2, 1>(x, wt, y, B, H, W, Cin, Cout, st) : cv::launch_v2<256, 1, 2>(x, wt, y, B, H, W, Cin, Cout, st);
-    if (Cout % 128 == 0) return m2 ? cv::launch_v2<128, 2, 2>(x, wt, y, B, H, W, Cin, Cout, st) : cv::launch_v2<128, 1, 2>(x, wt, y, B, H, W, Cin, Cout, st);
-    return m2 ? cv::launch_v2<64, 2, 2>(x, wt, y, B, H, W, Cin, Cout, st) : cv::launch_v2<64, 1, 2>(x, wt, y, B, H, W, Cin, Cout, st);
-  }
-  static const int force_mt = []() { const char* e = getenv("GF_CONV_MT"); return e ? atoi(e) : 0; }();     // tuning aid, read once
-  const bool mt2 = (H % 16 == 0) && force_mt != 1 && t2 >= nsm;
-  static const int big_env = []() { const char* e = getenv("GF_CONV_BIG"); return e ? atoi(e) : -1; }();
-  const bool big = big_env >= 0 ? big_env != 0 : big_v1;
-  if (Cout % 256 == 0 && big && H % 16 == 0) return cv::launch<256, 2, 1>(x, wt, y, B, H, W, Cin, Cout, st);
-  if (Cout % 256 == 0 && force_mt != 2) return cv::launch<256, 1, 2>(x, wt, y, B, H, W, Cin, Cout, st);
-  if (Cout % 128 == 0) return mt2 ? cv::launch<128, 2, 2>(x, wt, y, B, H, W, Cin, Cout, st) : cv::launch<128, 1, 2>(x, wt, y, B, H, W, Cin, Cout, st);
-  return mt2 ? cv::launch<64, 2, 2>(x, wt, y, B, H, W, Cin, Cout, st) : cv::launch<64, 1, 2>(x, wt, y, B, H, W, Cin, Cout, st);
+  if (!v) v = cv::dispatch(B, H, W, Cin, Cout);
+  if ((rc = v->fn(x, wt, y, B, H, W, Cin, Cout, (cudaStream_t)stream))) return rc;
+  g_last_variant[0] = v->version; g_last_variant[1] = v->bn; g_last_variant[2] = v->mt;
+  return GF_OK;
+}
+
+extern "C" int gf_conv3x3_nhwc_tf32(const float* x, const float* wt, float* y, int B, int H, int W, int Cin, int Cout, void* stream) {
+  return gf_conv3x3_nhwc_tf32_ex(x, wt, y, B, H, W, Cin, Cout, 0, 0, 0, stream);
+}
+
+extern "C" int gf_conv3x3_last_variant(int* version, int* bn, int* mt) {
+  if (!version || !bn || !mt) { set_error("gf_conv3x3_last_variant: null pointer"); return GF_ERR_INVALID; }
+  *version = g_last_variant[0]; *bn = g_last_variant[1]; *mt = g_last_variant[2];
+  return GF_OK;
 }

@@ -330,14 +330,16 @@ def conv3x3_pack(weight: torch.Tensor, scale: float = 1.0) -> torch.Tensor:
     return wt
 
 
-def conv3x3_native(x: torch.Tensor, wt: torch.Tensor) -> torch.Tensor:
+def conv3x3_native(x: torch.Tensor, wt: torch.Tensor, variant: Optional[tuple] = None) -> torch.Tensor:
     """3x3 stride-1 zero-padded convolution on the tcgen05 implicit-GEMM kernel (row f1, TF32): x [B, I, H, W] (channels-last
-    storage), wt from conv3x3_pack -> [B, O, H, W] (channels-last storage).  CUDA fp32 inference only."""
+    storage), wt from conv3x3_pack -> [B, O, H, W] (channels-last storage).  CUDA fp32 inference only.
+    variant: (version, bn, mt) forces one kernel instantiation (gf_conv3x3_nhwc_tf32_ex); None = the shape dispatch."""
     xv = _nhwc_view(x)
     B, H, W, I = xv.shape
     O = wt.shape[1]
     y = torch.empty((B, H, W, O), dtype=torch.float32, device=x.device)
+    version, bn, mt = variant if variant is not None else (0, 0, 0)
     with torch.cuda.device(x.device):
-        _lib.check(_lib.load().gf_conv3x3_nhwc_tf32(xv.data_ptr(), wt.data_ptr(), y.data_ptr(), B, H, W, I, O, _stream(x.device)),
-                   "gf_conv3x3_nhwc_tf32")
+        _lib.check(_lib.load().gf_conv3x3_nhwc_tf32_ex(xv.data_ptr(), wt.data_ptr(), y.data_ptr(), B, H, W, I, O, version, bn, mt,
+                                                       _stream(x.device)), "gf_conv3x3_nhwc_tf32")
     return y.permute(0, 3, 1, 2)

@@ -95,6 +95,16 @@ int gf_mapping_fwd(const float* z, const float* w, const float* b, const float* 
 int gf_conv3x3_pack_weights(const float* w, float* wt, int Cout, int Cin, float scale, void* stream);
 int gf_conv3x3_nhwc_tf32(const float* x, const float* wt, float* y, int B, int H, int W, int Cin, int Cout, void* stream);
 
+/* gf_conv3x3_nhwc_tf32 on a chosen kernel instantiation: version 1 (one activation box per tap) or 2 (one box per filter column),
+ * bn = output channels per tile (64 / 128 / 256), mt = 8 x 16 patches stacked per tile (1 or 2); the accumulator count follows
+ * (one set for bn 256, mt 2, else two).  (0, 0, 0) = the shape dispatch of gf_conv3x3_nhwc_tf32, GF_CONV_* overrides included.
+ * Any other triple must be one of the twelve, with Cout % bn == 0 and H % (8 mt) == 0, else GF_ERR_UNSUPPORTED before any device
+ * work.  All instantiations of one version sum in the same order, so they give bit-identical results. */
+int gf_conv3x3_nhwc_tf32_ex(const float* x, const float* wt, float* y, int B, int H, int W, int Cin, int Cout,
+                            int version, int bn, int mt, void* stream);
+/* (version, bn, mt) of the kernel the last gf_conv3x3_nhwc_tf32[_ex] call on this host thread launched; zeros if that call failed. */
+int gf_conv3x3_last_variant(int* version, int* bn, int* mt);
+
 #ifdef __cplusplus
 }
 #endif

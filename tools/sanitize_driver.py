@@ -1,7 +1,7 @@
 """Small-shape driver for compute-sanitizer (tools/sanitize.sh): one launch of every tensor-path kernel family --
 token_tc_kernel single-pass (C = 128, fused post-op with both scales), two-pass (C = 512), short tiles (8x8 grid),
 centroid_tc_kernel (+ gemm_tc_kernel, merge) via duplex layers incl. the C = 512 channel-split -- plus the CUDA-core kernels
-(fp32 mode) and the stage-T backward.  Checks every output against the fp64 oracle so a sanitizer-clean run is also a
+(fp32 mode), the stage-T backward, and every instantiation of the 3x3 convolution kernel (SAN_ONLY=conv for those alone).  Checks every output against the fp64 oracle so a sanitizer-clean run is also a
 correct one."""
 import os, sys
 sys.path.insert(0, os.path.dirname(os.path.dirname(os.path.abspath(__file__))))
@@ -67,6 +67,21 @@ if not only or "conv" in only:
         r = ((got - ref).abs().max() / ref.abs().max()).item()
         print(f"conv3x3 B={B} {H}x{W} {ci}->{co} max rel err {r:.3e}", flush=True)
         bad += r > 3e-3
+    # each of the twelve instantiations once, forced through gf_conv3x3_nhwc_tf32_ex, on a grid of 2 x SMs + 2 tiles (every CTA
+    # runs two or three tiles: accumulator sets reused, barrier phases flipped)
+    nsm = torch.cuda.get_device_properties(dev).multi_processor_count
+    for v in (1, 2):
+        for bn in (256, 128, 64):
+            for mt in (2, 1):
+                B, H, W, ci, co = nsm + 1, 8 * mt, 32, 32, bn
+                x = torch.randn(B, ci, H, W, device=dev).contiguous(memory_format=torch.channels_last)
+                w = torch.randn(co, ci, 3, 3, device=dev) / (ci * 9) ** 0.5
+                got = ops.conv3x3_native(x, ops.conv3x3_pack(w), variant=(v, bn, mt))
+                ref = torch.nn.functional.conv2d(x, w, padding=1)
+                torch.cuda.synchronize()
+                r = ((got - ref).abs().max() / ref.abs().max()).item()
+                print(f"conv3x3 v{v} bn={bn} mt={mt} B={B} {H}x{W} {ci}->{co} tiles={2 * B} max rel err {r:.3e}", flush=True)
+                bad += r > 3e-3 or gf._lib.conv3x3_last_variant() != (v, bn, mt)
 # attention dropout (CUDA-core forward + backward with the Philox mask)
 if not only or "dropout" in only:
     attn = gf.BipartiteAttention(64, 16, 4, pos_dim=16, att_dp=0.2).to(dev).train()
